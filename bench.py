@@ -5,6 +5,7 @@ backward -> single gradient all-reduce -> Adam) of the speech Transformer, BASEL
 
     python bench.py --gpus N --steps K --warmup W                 # ours  (torchrun launches N>1)
     python bench.py --impl reference --gpus N --steps K --warmup W    # the reference algorithm on the host CPU
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR  # + the last timed step's outputs as DIR/*.npy
 
 Prints ONE JSON line (see the task contract): `value` = whole-job utt/s with inputs resident in HBM, `e2e` = the same
 step through the public API with pinned-host inputs copied in and the loss read back every step, `roofline` for the
@@ -306,6 +307,32 @@ def run_reference(args, rank, world):
 
 
 # ---------------------------------------------------------------------------------------------------- GPU arm
+DUMP_SAMPLE = 1 << 19        # elements of the parameter / gradient buffers written by --dump-outputs (fixed, seeded indices)
+DUMP_BYTES = 64 * 10 ** 6    # --dump-outputs writes at most this much in all
+
+
+def dump_outputs(out_dir, last, dp):
+    """What the last timed DataParallelStep.step handed back and left behind, as float32 / float64 .npy files (about 60 MB
+    at cfg2): pred [B, T_tgt, V] and hyp [B, T_tgt] as returned, the loss statistics [sum, n_tokens, n_correct, mean,
+    1 / n_tokens], the global loss, and a fixed sample of the updated parameters and of the gradients of that step.  A pred
+    that would take the total over DUMP_BYTES (--batch > 32) is written as `pred_sample`, a fixed sample of its elements."""
+    import numpy as np
+    pred, hyp, stats = last
+    flat = dp.flat
+    idx = torch.from_numpy(np.random.RandomState(0).randint(0, flat.numel, DUMP_SAMPLE)).to(flat.flat.device)
+    arrays = {"hyp": hyp.float(), "loss_stats": stats.double(), "global_loss": dp.global_loss().double(),
+              "params_sample": flat.flat[idx].float(), "grads_sample": flat.flat_grad[idx].float()}
+    room = (DUMP_BYTES - sum(t.numel() * t.element_size() for t in arrays.values()) - 4096) // 4      # float32 elements
+    if pred.numel() <= room:
+        arrays["pred"] = pred.float()
+    else:
+        pidx = torch.from_numpy(np.random.RandomState(1).randint(0, pred.numel(), room)).to(pred.device)
+        arrays["pred_sample"] = pred.reshape(-1)[pidx].float()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().numpy())
+
+
 def run_b200(args, rank, local_rank, world):
     import torch.distributed as dist
     import b200asr
@@ -358,9 +385,11 @@ def run_b200(args, rank, local_rank, world):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        dp.step(src_d, lens_d, tgt_d)
+        last = dp.step(src_d, lens_d, tgt_d)
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last, dp)
     launches = (lib.b200asr_launch_count() - launches0) / args.steps
     ms_dev = max_over_ranks(e0.elapsed_time(e1)) / args.steps
     # ---- forward + loss + backward alone (BASELINE.json's metric names fwd+bwd; `value` above is the whole step incl. the
@@ -519,7 +548,12 @@ def main():
     ap.add_argument("--precision", default="", help="linear,conv,attn[,conv_wgrad[,attn_bwd]] in {fp32,tf32,tf32x3} (default: package default)")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-ref-gpu", action="store_true", help="skip timing the unmodified reference eager on this GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (inputs and weights are seeded, so two "
+                         "builds can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

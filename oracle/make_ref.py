@@ -7,7 +7,8 @@ TEST INFRASTRUCTURE ONLY.  The reference is a pure-Python application (no setup.
 is copying the three packages the hot path imports -- models/, utils/, trainer/ (+ data/labels/*.json for the vocabularies)
 -- byte for byte from where they lie under /root/reference.  oracle/_ref/ is listed in .gitignore (the sources never enter
 this repository's history) and is NOT in .gpurunignore, so the `gpurun` snapshot carries it to the box, where
-  * tests/test_gpu_reference.py runs the unmodified reference classes on the B200 with and without b200asr.install(),
+  * tests/test_host_logic.py::test_install_rebinds_reference_classes_and_keeps_module_tree binds b200asr.install() onto
+    the unmodified reference classes (tests/test_gpu_reference.py compares with stored reference results instead),
   * bench.py --impl reference times the reference's own CPU path, and bench.py's `reference_gpu` object times the
     reference eager on the same B200.
 Nothing in the product package imports from here.  `__graft_entry__.build()` calls stage() when /root/reference exists.

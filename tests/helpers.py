@@ -89,6 +89,53 @@ def assert_grads_close(grads: dict, ref: dict, tol: float, exact_kernels: bool):
         assert float((g - r.double()).norm()) / denom < 10 * tol, k
 
 
+def sample_index(numel: int, n: int, seed: int) -> np.ndarray:
+    """Fixed flat indices of a large tensor that a fixture stores a sample of (numpy's legacy generator: a stable stream)."""
+    if numel <= n:
+        return np.arange(numel)
+    return np.random.RandomState(seed).randint(0, numel, n)
+
+
+def reference_batch(B, freq, T, vocab, Lt, seed=0):
+    """Ragged, length-sorted synthetic batch (src [B,1,freq,T] zero past each length, int32 lengths, PAD-padded targets
+    and their int32 lengths), in the shape utils/data_loader.py's _collate_fn hands it over."""
+    g = torch.Generator().manual_seed(seed)
+    src = torch.randn(B, 1, freq, T, generator=g)
+    lens = (T * (0.5 + 0.5 * torch.rand(B, generator=g))).long().clamp(1, T)
+    lens[0] = T
+    lens = torch.sort(lens, descending=True).values
+    for i in range(B):
+        src[i, :, :, int(lens[i]):] = 0
+    tgt = torch.randint(3, vocab, (B, Lt), generator=g)
+    tl = (Lt * (0.4 + 0.6 * torch.rand(B, generator=g))).long().clamp(1, Lt)
+    tl[0] = Lt
+    for i in range(B):
+        tgt[i, int(tl[i]):] = 0
+    return src, lens.to(torch.int32), tgt, tl.to(torch.int32)
+
+
+def batch_checksum(src, lens, tgt) -> np.ndarray:
+    """Stored next to a regenerated batch so that a change of torch's random stream shows up as such."""
+    return np.array([float(src.double().sum()), float(src.double().abs().sum()), float(lens.sum()), float(tgt.sum())])
+
+
+def seeded_state(shapes: dict, seed: int) -> dict:
+    """Parameters regenerated from a seed instead of stored in a fixture: N(0, 1/fan_in) for matrices and convolution
+    kernels, 1 + N(0, 0.01) for 1-d weights (LayerNorm / BatchNorm scales), N(0, 0.01) for biases."""
+    out = {}
+    for i, (name, shape) in enumerate(sorted(shapes.items())):
+        r = np.random.RandomState(seed + i)
+        shape = tuple(shape)
+        if len(shape) >= 2:
+            v = r.standard_normal(shape) / np.sqrt(float(np.prod(shape[1:])))
+        elif name.endswith("weight"):
+            v = 1.0 + 0.1 * r.standard_normal(shape)
+        else:
+            v = 0.1 * r.standard_normal(shape)
+        out[name] = torch.from_numpy(v.astype(np.float32))
+    return out
+
+
 def load_greedy_golden():
     """tests/golden/greedy.npz: token ids of the reference's Decoder.greedy_search (cut at EOS), the encoder output fed to it
     and the decoder parameters (generated by tests/golden/make_golden.py::run_greedy from the live reference)."""

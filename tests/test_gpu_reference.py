@@ -1,36 +1,30 @@
-"""The UNMODIFIED reference on the B200, with and without `b200asr.install()` (SURVEY.md 8b: the drop-in boundary on hardware).
+"""The B200 path against the UNMODIFIED reference's own numbers (SURVEY.md 8b: the drop-in boundary on hardware).
 
-The reference checkout travels to the GPU box as oracle/_ref (staged by oracle/make_ref.py, git-ignored).  Here
-  * `init_transformer_model` (utils/functions.py:116-152) builds the reference's own `Transformer`;
-  * the SAME weights run (i) on the CPU, uninstalled -- the reference's own PyTorch forward/backward, (ii) on the GPU,
-    uninstalled -- the reference eager on the B200 (fp32 flags), (iii) on the GPU after `install()` -- our kernels bound onto
-    the reference's classes; pred / loss / num_correct / every gradient are compared;
-  * the reference's `Trainer.train` loop (trainer/asr/trainer.py:20-211) is driven unchanged for an epoch (train iterations
-    with `opt.step()` of the reference's NoamOpt + torch Adam, the eval-mode validation loop, the checkpoint save) with
-    synthetic `_collate_fn`-shaped batches, once on the reference eager and once installed: losses, updated parameters and
-    BatchNorm buffers must agree.
+The fixtures tests/golden/ref_<case>.npz and trainer_<case>.npz were written by tests/golden/make_golden.py from the
+reference itself on the CPU; parameters (helpers.seeded_state) and input batches (helpers.reference_batch) are
+regenerated here from their seeds, and arrays of more than a few thousand elements are stored as a fixed sample with the
+whole array's max |x| and L2 norm (cfg2_arch alone has 37M gradient elements and 12M front-end units):
+  * ref_<case>: the reference's `Transformer` (utils/functions.py:116-152) forward / calculate_metrics / backward -- pred,
+    gold, hyp, loss, num_correct, every gradient and the branch every ReLU / Hardtanh unit took;
+  * trainer_<case>: one epoch of the reference's `Trainer.train` loop (trainer/asr/trainer.py:20-211): 3 training
+    iterations with NoamOpt + torch Adam and gradient clipping, then the eval-mode validation batch -- the loss of every
+    iteration, the learning rate of every step and the change of every parameter and BatchNorm buffer.
+Our model is the state_dict-compatible mirror (b200asr.build_model) running on the CUDA kernels.
 """
-import copy
-import os
 import importlib
-import tempfile
+import os
 
+import numpy as np
 import pytest
 import torch
 
-from oracle import ref_shim
-from tests.helpers import grads_rel_err, rel_err
+from oracle import asr_oracle as O
+from tests.gpu_util import cuda_model
+from tests.helpers import GOLDEN_DIR, batch_checksum, reference_batch, sample_index, seeded_state
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not ref_shim.available(), reason="reference checkout not staged (oracle/make_ref.py)")]
+pytestmark = pytest.mark.gpu
 
 TOL = 1e-3
-
-SMALL_VGG = ["--num-layers", "2", "--num-heads", "2", "--dim-model", "64", "--dim-emb", "64", "--dim-key", "32", "--dim-value", "32",
-             "--dim-inner", "128", "--feat_extractor", "vgg_cnn", "--sample-rate", "4000", "--tgt-max-len", "12"]
-SMALL_EMB = ["--num-layers", "1", "--num-heads", "2", "--dim-model", "64", "--dim-emb", "64", "--dim-key", "32", "--dim-value", "32",
-             "--dim-inner", "128", "--feat_extractor", "emb_cnn", "--tgt-max-len", "10"]
-CFG2_ARCH = ["--num-layers", "4", "--num-heads", "8", "--dim-model", "512", "--dim-emb", "512", "--dim-key", "64", "--dim-value", "64",
-             "--dim-inner", "2048", "--feat_extractor", "vgg_cnn", "--tgt-max-len", "40"]
 
 
 def _fp32_flags():
@@ -38,33 +32,65 @@ def _fp32_flags():
     torch.backends.cuda.matmul.allow_tf32 = False
 
 
-def _build(flags, vocab, extra=()):
-    ns = ref_shim.load(list(flags) + ["--dropout", "0.0", "--label-smoothing", "0.1"] + list(extra))
-    l2i, i2l = ref_shim.labels(vocab)
-    torch.manual_seed(123456)
-    model = ns.functions.init_transformer_model(ns.constant.args, l2i, i2l)
-    g = torch.Generator().manual_seed(7)
-    with torch.no_grad():
-        for p in model.parameters():
-            if p.dim() == 1:
-                p.add_(0.1 * torch.randn(p.shape, generator=g))
-    return ns, model, l2i, i2l
+def _fixture(name):
+    z = np.load(os.path.join(GOLDEN_DIR, name + ".npz"))
+    c = z["meta.cfg"]
+    cfg = O.OracleConfig(num_layers=int(c[0]), num_heads=int(c[1]), dim_model=int(c[2]), dim_key=int(c[3]),
+                         dim_value=int(c[4]), dim_inner=int(c[5]), vocab=int(c[6]), tgt_max_len=int(c[7]),
+                         freq=int(c[8]), feat_extractor=str(z["meta.feat"]))
+    return z, cfg
 
 
-def _batch(B, freq, T, vocab, Lt, seed=0, ragged=True):
-    g = torch.Generator().manual_seed(seed)
-    src = torch.randn(B, 1, freq, T, generator=g)
-    lens = (T * (0.5 + 0.5 * torch.rand(B, generator=g))).long().clamp(1, T) if ragged else torch.full((B,), T)
-    lens[0] = T
-    lens = torch.sort(lens, descending=True).values
-    for i in range(B):
-        src[i, :, :, int(lens[i]):] = 0
-    tgt = torch.randint(3, vocab, (B, Lt), generator=g)
-    tl = (Lt * (0.4 + 0.6 * torch.rand(B, generator=g))).long().clamp(1, Lt)
-    tl[0] = Lt
-    for i in range(B):
-        tgt[i, int(tl[i]):] = 0
-    return src, lens.to(torch.int32), tgt, tl.to(torch.int32)
+def _model(z, cfg, train=True):
+    """The mirror model with the fixture's seeded parameters (BatchNorm buffers at their initial values)."""
+    import b200asr
+    from tests.gpu_util import asr_cfg
+    shapes = {n: p.shape for n, p in b200asr.build_model(asr_cfg(cfg)).named_parameters()}
+    return cuda_model(cfg, seeded_state(shapes, int(z["meta.seeded_state"])), train=train)
+
+
+def _batch(z, cfg, seed, checksum):
+    """The fixture's input batch, regenerated from its seed (helpers.reference_batch) and checked against its checksum."""
+    B, T = (int(v) for v in z["in.shape"])
+    src, lens, tgt, _ = reference_batch(B, cfg.freq, T, cfg.vocab, cfg.tgt_max_len - 1, seed=seed)
+    assert np.allclose(batch_checksum(src, lens, tgt), checksum, rtol=1e-9, atol=0), "torch's random stream changed"
+    return src, lens, tgt
+
+
+class Stored:
+    """One array of a fixture group (make_golden._pack): whole, or a fixed sample at helpers.sample_index, with the whole
+    array's shape, max |x| and L2 norm."""
+
+    def __init__(self, values, row):
+        seed, self.absmax, self.norm, off, count, ndim = (float(v) for v in row[:6])
+        self.shape = tuple(int(s) for s in row[6:6 + int(ndim)])
+        self.numel = int(np.prod(self.shape))
+        self.ref = torch.from_numpy(values[int(off):int(off) + int(count)])
+        self.idx = None if seed < 0 else torch.from_numpy(sample_index(self.numel, int(count), int(seed)))
+
+    def pick(self, t):
+        t = t.detach().cpu().reshape(-1)
+        return t if self.idx is None else t[self.idx]
+
+    def max_err(self, t):
+        """max |t - ref| over the stored elements."""
+        return float((self.pick(t).double() - self.ref.double()).abs().max())
+
+    def l2_err(self, t):
+        """|t - ref|_2 (estimated from the sample when only a sample is stored)."""
+        d = self.pick(t).double() - self.ref.double()
+        return float(d.norm()) * ((self.numel / d.numel()) ** 0.5 if self.idx is not None else 1.0)
+
+    def whole_errs(self, t):
+        """(| max|t| - max|ref| |, | |t|_2 - |ref|_2 |) over EVERY element: lower bounds of the max-norm and L2 errors that
+        also see the elements a sample leaves out."""
+        t = t.detach().double().cpu()
+        return abs(float(t.abs().max()) - self.absmax), abs(float(t.norm()) - self.norm)
+
+
+def _group(z, name):
+    values, info = z[name + ".values"], z[name + ".info"]
+    return {str(n): Stored(values, row) for n, row in zip(z[name + ".names"], info)}
 
 
 def _region(kind, t):
@@ -73,183 +99,145 @@ def _region(kind, t):
     return (t > 0).to(torch.int8) + ((t >= 20).to(torch.int8) if kind == "hardtanh" else 0)
 
 
-class _RefDecisions:
-    """Forward hooks on the UNMODIFIED reference: the branch taken by every Hardtanh / ReLU unit of the CNN front end and by
-    every ReLU of the position-wise FFNs (F.relu there: hooked through conv_1's output), in execution order -- the order in
-    which ops.decision_capture lists the same units of our path (its max-pool entries have no counterpart here)."""
-
-    def __init__(self, model):
-        self.out, self.handles = [], []
-        for m in model.modules():
-            if isinstance(m, torch.nn.Hardtanh):
-                self.handles.append(m.register_forward_hook(lambda _m, _i, o: self.out.append(_region("hardtanh", o))))
-            elif isinstance(m, torch.nn.ReLU):
-                self.handles.append(m.register_forward_hook(lambda _m, _i, o: self.out.append(_region("relu", o))))
-            elif type(m).__name__ == "PositionwiseFeedForwardWithConv":      # conv_1 output is [B, d_inner, T]
-                self.handles.append(m.conv_1.register_forward_hook(lambda _m, _i, o: self.out.append(_region("relu", o.transpose(1, 2)))))
-
-    def close(self):
-        for h in self.handles:
-            h.remove()
-        return self.out
-
-
-def _count_flips(ref, ours):
-    """(# units whose branch differs, # units); None if the two lists do not describe the same units."""
+def _count_flips(z, ours):
+    """(# units whose branch differs, # units compared); None if the two lists do not describe the same units.  The
+    fixture lists the reference's ReLU / Hardtanh units (and the FFNs' F.relu) in execution order, the order in which
+    ops.decision_capture lists the same units of our path (its max-pool entries have no counterpart there)."""
     ours = [_region(k, t) for k, t in ours if k != "pool"]
-    if len(ours) != len(ref) or any(a.shape != b.shape for a, b in zip(ours, ref)):
+    refs = _group(z, "dec")
+    if len(ours) != len(refs):
         return None
-    return sum(int((a != b).sum()) for a, b in zip(ours, ref)), sum(a.numel() for a in ref)
-
-
-def _step(ns, model, src, lens, tgt, dev, decisions=None):
-    """One forward / loss / backward through the reference's own code.  decisions: "hooks" records the branch decisions of the
-    (uninstalled) reference, "capture" those of our kernels; they are returned as the seventh element."""
-    import b200asr
-    ops = importlib.import_module(b200asr.__name__ + ".ops")
-    model.zero_grad(set_to_none=True)
-    rec = _RefDecisions(model) if decisions == "hooks" else None
-    if decisions == "capture":
-        ops.decision_capture = []
-    try:
-        pred, gold, hyp, _ = model(src.to(dev), lens, tgt.to(dev), verbose=False)
-    finally:
-        dec = rec.close() if rec else ops.decision_capture
-        ops.decision_capture = None
-    loss, n_correct = ns.metrics.calculate_metrics(pred, gold, smoothing=0.1, loss_type="ce")
-    loss.backward()
-    grads = {n: p.grad.detach().float().cpu() for n, p in model.named_parameters()}
-    return pred.detach().float().cpu(), gold.cpu(), hyp.cpu(), float(loss.item()), int(n_correct), grads, dec
+    flips = units = 0
+    for i, t in enumerate(ours):
+        ref = refs[str(i)]
+        if tuple(t.shape) != ref.shape:
+            return None
+        flips += int((ref.pick(t) != ref.ref).sum())
+        units += ref.ref.numel()
+    return flips, units
 
 
 @pytest.mark.parametrize("case", ["small_vgg", "small_emb", "cfg2_arch"])
-def test_install_on_unmodified_reference_matches_reference_forward_backward(case):
+def test_matches_reference_forward_backward(case):
     import b200asr
-    flags, vocab, freq, B, T = {"small_vgg": (SMALL_VGG, 40, 41, 3, 32), "small_emb": (SMALL_EMB, 40, 161, 3, 48),
-                                "cfg2_arch": (CFG2_ARCH, 4364, 161, 2, 200)}[case]
-    ns, model, _, _ = _build(flags, vocab)
-    src, lens, tgt, _ = _batch(B, freq, T, vocab, ns.constant.args.tgt_max_len - 1)
-    keys = list(model.state_dict().keys())
-    model.train()
+    ops = importlib.import_module(b200asr.__name__ + ".ops")
+    z, cfg = _fixture("ref_" + case)
     _fp32_flags()
-    cpu = _step(ns, model, src, lens, tgt, "cpu", "hooks")              # (i) the reference's own CPU forward/backward
-    model = model.cuda()
-    eager = _step(ns, model, src, lens, tgt, "cuda", "hooks")           # (ii) the reference eager on the B200
-    orig_forward = ns.transformer.Transformer.forward
-    b200asr.install()
+    model = _model(z, cfg)
+    src, lens, tgt = _batch(z, cfg, int(z["in.seed"]), z["in.checksum"])
+    launches0 = b200asr._lib.load().b200asr_launch_count()
+    model.zero_grad(set_to_none=True)
+    ops.decision_capture = []
     try:
-        assert ns.transformer.Transformer.forward is not orig_forward
-        launches0 = b200asr._lib.load().b200asr_launch_count()
-        ours = _step(ns, model, src, lens, tgt, "cuda", "capture")      # (iii) our kernels behind the reference's classes
-        assert b200asr._lib.load().b200asr_launch_count() > launches0   # ... and they did launch
+        pred, gold, hyp, _ = model(src.cuda(), lens, tgt.cuda())
+        dec = ops.decision_capture
     finally:
-        b200asr.uninstall()
-    assert ns.transformer.Transformer.forward is orig_forward
-    assert list(model.state_dict().keys()) == keys                      # module tree / parameter names untouched
-    for name, other in (("cpu", cpu), ("eager-gpu", eager)):
-        assert torch.equal(ours[1], other[1]), name                     # gold
-        e_pred = rel_err(ours[0], other[0])
-        errs = grads_rel_err(ours[5], other[5])
-        worst = max(errs, key=errs.get)
-        real = other[1].ne(0)
-        flips = int((ours[2][real] != other[2][real]).sum())
-        print(f"[{case}] installed vs {name}: pred {e_pred:.2e} loss {abs(ours[3] - other[3]) / abs(other[3]):.2e} "
-              f"grads max {errs[worst]:.2e} ({worst}) argmax flips {flips}/{int(real.sum())} num_correct {ours[4]} vs {other[4]}")
-        assert e_pred < TOL
-        assert abs(ours[3] - other[3]) < TOL * abs(other[3])
-        # 1e5 .. 1e7 ReLU / max-pool units: a handful sit within rounding of their threshold and decide differently under two
-        # correct arithmetics (the reference's CPU and GPU runs differ from each other the same way), which moves single
-        # rows of the token-sparse decoder FFN gradients by O(1/sqrt(tokens)).  The strict max-norm check of EVERY gradient
-        # at the path's own decisions lives in tests/test_gpu_fullsize_parity.py (the oracle there is pinned bit-exactly to
-        # this reference, where decisions can be frozen); here: the median tensor in the max norm, every tensor in the
-        # relative L2 norm.
-        med = sorted(errs.values())[len(errs) // 2]
-        unit_flips = _count_flips(other[6], ours[6])
-        print(f"[{case}] installed vs {name}: ReLU / Hardtanh units that took another branch: {unit_flips}")
-        assert unit_flips is not None, "decision lists of the reference hooks and of ops.decision_capture do not line up"
-        # every unit on the same branch: tight bounds.  Otherwise (k of ~1e5 .. 1e7 units within rounding of their threshold):
-        # a flipped FFN unit adds / removes one token's term in ITS row of that layer's weight gradient (relative L2 of the
-        # tensor up to ~1/sqrt(d_inner)) and moves the gradients below it by O(1 / (tokens sqrt(d_inner))): bounded, not exact.
-        same = unit_flips[0] == 0
-        assert unit_flips[0] <= 2 + unit_flips[1] // 100000, (name, unit_flips)
-        assert med < ((5 if case == "cfg2_arch" else 1) * TOL if same else 10 * TOL), (name, med, unit_flips)
-        for k, r in other[5].items():
-            denom = max(float(r.norm()), 1e-3 * max(float(v.abs().max()) for v in other[5].values()) * r.numel() ** 0.5)
-            assert float((ours[5][k] - r).norm()) / denom < (10 * TOL if same else 0.2), (name, k, unit_flips)
-        assert flips <= max(1, int(real.sum()) // 100)                  # near-ties at random init
-        assert abs(ours[4] - other[4]) <= max(1, int(real.sum()) // 100)
+        ops.decision_capture = None
+    loss, n_correct = b200asr.calculate_metrics(pred, gold, smoothing=0.1)
+    loss.backward()
+    torch.cuda.synchronize()
+    assert b200asr._lib.load().b200asr_launch_count() > launches0          # our kernels ran
+    grads = {n: p.grad for n, p in model.named_parameters()}
 
-
-def _loaders(freq, T, vocab, Lt, n_train, B):
-    def one(seed):
-        src, lens, tgt, tl = _batch(B, freq, T, vocab, Lt, seed=seed)
-        return (src, tgt, lens.float() / float(T), lens, tl)            # _collate_fn order, utils/data_loader.py:213
-    return [one(s) for s in range(n_train)], [[one(100)]]
-
-
-def _run_trainer(ns, model, l2i, i2l, train, valid, installed, tmp):
-    """Drive the reference's Trainer.train unchanged for one epoch; returns (per-iteration losses, state_dict)."""
-    import b200asr
-    ns.constant.args.save_folder, ns.constant.args.name = tmp, "b200" if installed else "eager"
-    opt = ns.functions.init_optimizer(ns.constant.args, model, "noam")
-    losses = []
-    if installed:
-        b200asr.install()
-    cur = ns.trainer.calculate_metrics
-
-    def recording(*a, **k):
-        out = cur(*a, **k)
-        losses.append(float(out[0].item()))
-        return out
-
-    ns.trainer.calculate_metrics = recording
-    try:
-        tr = copy.deepcopy(train), copy.deepcopy(valid)                 # the loop scales src_percentages in place (trainer.py:82)
-        ns.trainer.Trainer().train(model, tr[0], None, tr[1], opt, "ce", 0, 1, l2i, i2l)
-    finally:
-        ns.trainer.calculate_metrics = cur
-        if installed:
-            b200asr.uninstall()
-    assert os.path.exists(os.path.join(tmp, ns.constant.args.name, "best_model.th"))      # save_model ran (functions.py:10-57)
-    return losses, {k: v.detach().float().cpu().clone() for k, v in model.state_dict().items()}
+    gold_r, hyp_r = torch.from_numpy(z["out.gold"]), torch.from_numpy(z["out.hyp"])
+    loss_r, nc_r = float(z["out.loss"]), int(z["out.num_correct"])
+    assert torch.equal(gold.cpu(), gold_r)
+    p_ref = _group(z, "pred")["pred"]
+    e_pred = p_ref.max_err(pred) / p_ref.absmax
+    ref_g = _group(z, "grad")
+    assert set(ref_g) == set(grads)
+    gmax = max(r.absmax for r in ref_g.values())
+    errs = {n: r.max_err(grads[n]) / max(r.absmax, 1e-3 * gmax) for n, r in ref_g.items()}
+    worst = max(errs, key=errs.get)
+    real = gold_r.ne(0)
+    flips = int((hyp.cpu()[real] != hyp_r[real]).sum())
+    print(f"[{case}] vs reference: pred {e_pred:.2e} loss {abs(loss.item() - loss_r) / abs(loss_r):.2e} "
+          f"grads max {errs[worst]:.2e} ({worst}) argmax flips {flips}/{int(real.sum())} num_correct {n_correct} vs {nc_r}")
+    assert e_pred < TOL
+    assert abs(loss.item() - loss_r) < TOL * abs(loss_r)
+    # 1e5 .. 1e7 ReLU / max-pool units: a handful sit within rounding of their threshold and decide differently under two
+    # correct arithmetics (the reference's CPU and GPU runs differ from each other the same way), which moves single
+    # rows of the token-sparse decoder FFN gradients by O(1/sqrt(tokens)).  The strict max-norm check of EVERY gradient
+    # at the path's own decisions lives in tests/test_gpu_fullsize_parity.py (the oracle there is pinned bit-exactly to
+    # this reference, where decisions can be frozen); here: the median tensor in the max norm, every tensor in the
+    # relative L2 norm.
+    med = sorted(errs.values())[len(errs) // 2]
+    unit_flips = _count_flips(z, dec)
+    print(f"[{case}] vs reference: ReLU / Hardtanh units that took another branch: {unit_flips}")
+    assert unit_flips is not None, "decision lists of the reference fixture and of ops.decision_capture do not line up"
+    # every unit on the same branch: tight bounds.  Otherwise (k of ~1e5 .. 1e7 units within rounding of their threshold):
+    # a flipped FFN unit adds / removes one token's term in ITS row of that layer's weight gradient (relative L2 of the
+    # tensor up to ~1/sqrt(d_inner)) and moves the gradients below it by O(1 / (tokens sqrt(d_inner))): bounded, not exact.
+    # The count covers the stored units only (a fixed sample of the large front-end layers), so `same` can hold while an
+    # unsampled unit flipped; the tight bounds then apply where the relaxed ones would be due.  That errs towards a false
+    # failure, never a false pass: if one appears after a kernel change, check the flips on the whole layers first.
+    same = unit_flips[0] == 0
+    assert unit_flips[0] <= 2 + unit_flips[1] // 100000, unit_flips
+    assert med < ((5 if case == "cfg2_arch" else 1) * TOL if same else 10 * TOL), (med, unit_flips)
+    for n, r in ref_g.items():
+        denom = max(r.norm, 1e-3 * gmax * r.numel ** 0.5)
+        bound = 10 * TOL if same else 0.2
+        assert r.l2_err(grads[n]) / denom < bound, (n, unit_flips)
+        d_max, d_l2 = r.whole_errs(grads[n])
+        assert d_l2 / denom < bound and d_max / max(r.absmax, 1e-3 * gmax) < bound, (n, d_max, d_l2, unit_flips)
+    assert flips <= max(1, int(real.sum()) // 100)                      # near-ties at random init
+    assert abs(n_correct - nc_r) <= max(1, int(real.sum()) // 100)
 
 
 @pytest.mark.parametrize("case", ["small_vgg", "small_emb"])
-def test_reference_trainer_loop_runs_on_installed_kernels(case):
-    """trainer/asr/trainer.py:47-118 (train) and :123-190 (eval-mode validation) -- unchanged code, our kernels underneath.
+def test_training_loop_matches_reference_trainer(case):
+    """trainer/asr/trainer.py:47-118 (train) and :123-190 (eval-mode validation) step for step: zero_grad -> forward ->
+    calculate_metrics -> backward -> clip_grad_norm_ -> Adam at the reference's NoamOpt rate, then the validation forward.
     small_emb also checks the BatchNorm buffers (running_mean / running_var / num_batches_tracked) and the eval-mode
     forward that uses them."""
-    flags, vocab, freq, B, T = {"small_vgg": (SMALL_VGG, 40, 41, 4, 32), "small_emb": (SMALL_EMB, 40, 161, 4, 48)}[case]
+    import b200asr
+    z, cfg = _fixture("trainer_" + case)
     _fp32_flags()
-    results = {}
-    with tempfile.TemporaryDirectory() as tmp:
-        for installed in (False, True):
-            ns, model, l2i, i2l = _build(flags, vocab, extra=["--cuda", "--warmup", "4", "--k-lr", "0.02", "--min-lr", "1e-6", "--clip", "--max-norm", "400"])
-            init = {k: v.detach().float().clone() for k, v in model.state_dict().items()}
-            if case == "small_emb":
-                # a conv bias in front of BatchNorm is a gauge freedom: its true gradient is zero, Adam turns the rounding noise
-                # into +-lr steps, and running_mean absorbs the resulting random walk.  Freeze it so the buffers are comparable.
-                model.conv[0].bias.requires_grad_(False)
-                model.conv[3].bias.requires_grad_(False)
-            model = model.cuda()
-            train, valid = _loaders(freq, T, vocab, ns.constant.args.tgt_max_len - 1, 3, B)
-            results[installed] = _run_trainer(ns, model, l2i, i2l, train, valid, installed, tmp)
-    (l_e, sd_e), (l_b, sd_b) = results[False], results[True]
-    print(f"[{case}] losses eager {l_e}\n[{case}] losses b200  {l_b}")
-    assert len(l_e) == len(l_b) == 4                                    # 3 train iterations + 1 validation batch
-    for a, b in zip(l_e, l_b):
-        assert abs(a - b) < TOL * abs(a), (l_e, l_b)
-    for k in sd_e:
+    model = _model(z, cfg)
+    for n in z["meta.frozen"]:
+        model.get_parameter(str(n)).requires_grad_(False)
+    init = {k: v.detach().float().cpu().clone() for k, v in model.state_dict().items()}
+    opt = torch.optim.Adam(model.parameters(), betas=(0.9, 0.98), eps=1e-9)       # utils/functions.py:107
+    rates = z["out.rates"]
+    losses = []
+    seeds = [int(s) for s in z["in.train.seeds"]] + [int(z["in.valid.seed"])]
+    batches = [_batch(z, cfg, s, c) for s, c in zip(seeds, z["in.checksum"])]
+    for j, (src, lens, tgt) in enumerate(batches[:-1]):
+        opt.zero_grad()
+        pred, gold, _, _ = model(src.cuda(), lens, tgt.cuda())
+        loss, _ = b200asr.calculate_metrics(pred, gold, smoothing=0.1)
+        losses.append(float(loss.item()))
+        loss.backward()
+        torch.nn.utils.clip_grad_norm_(model.parameters(), float(z["meta.max_norm"]))
+        for g in opt.param_groups:
+            g["lr"] = float(rates[j])
+        opt.step()
+    model.eval()
+    src, lens, tgt = batches[-1]
+    with torch.no_grad():
+        pred, gold, _, _ = model(src.cuda(), lens, tgt.cuda())
+        losses.append(float(b200asr.calculate_metrics(pred, gold, smoothing=0.1)[0].item()))
+    l_e = [float(v) for v in z["out.losses"]]
+    print(f"[{case}] losses reference {l_e}\n[{case}] losses b200      {losses}")
+    assert len(l_e) == len(losses) == 4                                 # 3 train iterations + 1 validation batch
+    for a, b in zip(l_e, losses):
+        assert abs(a - b) < TOL * abs(a), (l_e, losses)
+    sd = {k: v.detach().float().cpu() for k, v in model.state_dict().items()}
+    deltas = _group(z, "delta")
+    for k in sd:
         if "num_batches_tracked" in k:
-            assert sd_e[k].item() == sd_b[k].item() == 3, k
+            assert int(z["final." + k]) == sd[k].item() == 3, k
             continue
         if "running_" in k:
-            assert rel_err(sd_b[k], sd_e[k]) < TOL, k
+            r = torch.from_numpy(z["final." + k])
+            assert float((sd[k] - r).abs().max() / r.abs().max()) < TOL, k
             continue
         if k.endswith("positional_encoding.pe"):
             continue
-        d_e, d_b = sd_e[k] - init[k], sd_b[k] - init[k]
-        if d_e.numel() < 256:
+        d_e = deltas[k]
+        if d_e.numel < 256:
             continue                                                    # tiny tensors: Adam's sign-like first steps on noise-level gradients
         # Adam normalises the step, so an element whose gradient is rounding noise moves by +-lr either way: compare in L2
-        assert float((d_e - d_b).norm() / d_e.norm().clamp_min(1e-30)) < (0.05 if d_e.numel() >= 16384 else 0.15), k
+        bound = 0.05 if d_e.numel >= 16384 else 0.15
+        assert d_e.l2_err(sd[k] - init[k]) / max(d_e.norm, 1e-30) < bound, k
+        assert d_e.whole_errs(sd[k] - init[k])[1] / max(d_e.norm, 1e-30) < bound, k

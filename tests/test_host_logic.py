@@ -10,6 +10,7 @@ import torch
 
 import b200asr
 from oracle import asr_oracle as O
+from oracle import ref_shim
 from tests.helpers import GOLDEN_CASES, load_golden
 
 
@@ -96,10 +97,10 @@ def test_cpu_tensors_are_rejected_not_computed():
         b200asr.calculate_metrics(torch.randn(2, 3, 8), torch.ones(2, 3, dtype=torch.long))
 
 
-REF = "/root/reference"
+REF = ref_shim.reference_root()
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout only exists in the build container")
+@pytest.mark.skipif(REF is None, reason="no reference checkout: neither $B200ASR_REFERENCE nor oracle/_ref (staged by build())")
 def test_install_rebinds_reference_classes_and_keeps_module_tree():
     """Runs in a subprocess because the reference parses flags at import (utils/constant.py:99)."""
     import subprocess

@@ -23,7 +23,14 @@ def test_forward_loss_and_grads_match_reference(case):
     assert abs(loss.item() - io["out.loss"].item()) < 2e-5 * abs(io["out.loss"].item())
     assert O.num_correct(pred, gold) == int(io["out.num_correct"])
     assert set(G) == set(grads)
-    errs = grads_rel_err(grads, G)
+    # a convolution bias followed by training-mode BatchNorm (emb_cnn: conv.0 -> BN conv.1, conv.3 -> BN conv.4) cancels in
+    # the batch mean: its gradient is exactly zero, and both the fixture's and the oracle's values are rounding noise whose
+    # pattern depends on the CPU's thread count.  Those tensors must be zero to rounding; every other one must match.
+    gmax = max(float(v.abs().max()) for v in G.values())
+    gauge = [k for k in ("conv.0.bias", "conv.3.bias") if cfg.feat_extractor == "emb_cnn"]
+    for k in gauge:
+        assert float(G[k].abs().max()) < 1e-5 * gmax and float(grads[k].abs().max()) < 1e-5 * gmax, k
+    errs = {k: v for k, v in grads_rel_err(grads, G).items() if k not in gauge}
     worst = max(errs, key=errs.get)
     assert errs[worst] < 5e-4, (worst, errs[worst])
 
